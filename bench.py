@@ -28,6 +28,7 @@ import time
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(ROOT, "tests"))
+sys.dont_write_bytecode = True      # the benchmark leaves the source tree as it found it (it may be read-only)
 
 import numpy as np  # noqa: E402
 
@@ -112,18 +113,32 @@ def host_threads():
         return os.cpu_count() or 1
 
 
+def dump_outputs(out_dir, proof):
+    """Writes a proof (log_trace_heights bytes, fields u64[], commitments u64[n, 4]) as DIR/<name>.npy in float64.
+    Goldilocks elements do not fit a float64 mantissa, so every u64 becomes its [low, high] 32-bit halves (a trailing
+    axis of 2), which float64 holds exactly: two builds can then be compared value for value."""
+    heights, fields, comms = proof
+
+    def halves(a):
+        a = np.ascontiguousarray(a, dtype=np.uint64)
+        return np.stack([a & np.uint64(0xFFFFFFFF), a >> np.uint64(32)], axis=-1).astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "log_trace_heights.npy"), np.frombuffer(bytes(heights), dtype=np.uint8).astype(np.float64))
+    np.save(os.path.join(out_dir, "fields.npy"), halves(fields))
+    np.save(os.path.join(out_dir, "commitments.npy"), halves(comms))
+
+
 def cpu_baseline(log_height, steps=1, warmup=0, budget_s=None, hash_name="poseidon2"):
     """The oracle (C++ restatement of the reference prover, OpenMP over all host threads) proving the same workload
     shape.  With `budget_s` the number of timed proofs is cut (never below 1) so that the run ends inside the budget;
-    the number actually timed is returned and reported."""
+    the number actually timed is returned and reported, and so is the proof of the last timed run."""
     n_thr = host_threads()
     os.environ["OMP_NUM_THREADS"] = str(n_thr)      # before libgomp initialises
     os.environ.setdefault("OMP_WAIT_POLICY", "PASSIVE")   # the GPU hosts are shared: spinning at barriers collapses when a neighbour takes cores
     os.environ.pop("OMP_THREAD_LIMIT", None)
     import helpers as H
     import oracle_binding as ob
-    ob.build()
-    n_thr = ob.lib().orc_set_threads(n_thr)
+    n_thr = ob.lib().orc_set_threads(n_thr)      # build() made oracle/liboracle.so; no make here, the tree may be read-only
     W = H.W
     params = W.miden_pcs_params()
     wl = W.Workload([log_height] * 3)
@@ -141,6 +156,7 @@ def cpu_baseline(log_height, steps=1, warmup=0, budget_s=None, hash_name="poseid
         ob.lib().orc_prove_free(h)
         if i >= warmup:
             times.append(dt)
+            last_proof = (heights, fields, comms)
         i += 1
         if budget_s is not None:
             left = budget_s - (time.perf_counter() - t_start)
@@ -152,7 +168,7 @@ def cpu_baseline(log_height, steps=1, warmup=0, budget_s=None, hash_name="poseid
     mean = sum(times) / len(times)
     return {"value": wl.cells / mean, "unit": UNIT, "cores": n_thr, "kind": "port",
             "sample": f"synthetic 2^{log_height} x (51,22,16), full prove, {len(times)} timed run(s) after {warmup} warm-up, {mean:.2f} s each, "
-                      f"{n_thr} OpenMP threads (nproc {os.cpu_count()})"}, mean, wl.cells, len(times), warmup
+                      f"{n_thr} OpenMP threads (nproc {os.cpu_count()})"}, mean, wl.cells, len(times), warmup, last_proof
 
 
 def run_reference(args, rank):
@@ -163,7 +179,9 @@ def run_reference(args, rank):
         return
     lh = args.ref_log_height if args.ref_log_height else args.log_height
     budget = float(os.environ.get("MDN_REF_BUDGET_S", "600"))     # the driver killed the round-1 arm at ~820 s (per-N limit 870 s); leave room for start-up
-    cb, mean, cells, timed, warm = cpu_baseline(lh, steps=args.steps, warmup=min(args.warmup, 1), budget_s=budget, hash_name=args.hash)
+    cb, mean, cells, timed, warm, proof = cpu_baseline(lh, steps=args.steps, warmup=min(args.warmup, 1), budget_s=budget, hash_name=args.hash)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, proof)
     line = {
         "metric": METRIC, "value": cb["value"], "unit": UNIT, "n_gpus": args.gpus, "steps": timed, "warmup": warm,
         "ms_per_step": mean * 1e3, "higher_is_better": True, "scaling": "strong" if args.gpus > 1 else "weak", "vs_baseline": None, "dtype": "u64",
@@ -194,6 +212,10 @@ def main():
                     help="N>1: 'coset' (default) = ONE proof split over the GPUs -- LDE cosets, leaf sponge, constraints, DEEP and FRI "
                          "folds per coset, Merkle sub-trees per leaf range, peer-memory stores over NVLink (strong scaling); "
                          "'proof' = one independent proof per GPU (weak scaling, no data exchange)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the proof of the last timed step (rank 0's) as DIR/log_trace_heights.npy, "
+                         "DIR/fields.npy and DIR/commitments.npy in float64, each u64 as its [low, high] 32-bit halves; "
+                         "the inputs are seeded, so runs with the same arguments can be compared output for output")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl != "reference" else args.warmup
 
@@ -291,6 +313,8 @@ def main():
 
     total_v = pkg.parallel.max_over_ranks(total_v, "cuda")
     total_e = pkg.parallel.max_over_ranks(total_e, "cuda")
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, proof)      # the last step of the `value` region (device-resident traces)
 
     # Outside every timed region: the split proof must be the same bytes on every rank and the same bytes as the proof
     # of an unsplit single-GPU session (every rank proves it once as its local reference).
